@@ -15,6 +15,7 @@ scaling); one NCCL gather of the pose records at the end of the stream.
 
   python bench.py --gpus N --steps K --warmup W            # our arm (one process per GPU, torchrun for N > 1)
   python bench.py --impl reference --gpus N --steps K --warmup W   # reference arm: CPU path on the host cores
+  python bench.py --steps K --warmup W --dump-outputs DIR  # also write the poses of the last timed step as DIR/*.npy
 
 Prints ONE JSON line (rank 0). `value`: inputs resident in HBM. `e2e`: host (pinned) buffers in, pose records out,
 copies inside the timed region, through the public Python API. `precisions`: the same workload in the TF32 and the
@@ -23,6 +24,7 @@ C1 (SIFT + exact NN + 5-pt, 16 pairs), C3 (SuperPoint + SuperGlue + PnP), C4 (10
 ranks, strong scaling), C5 (RANSAC hypothesis sweep).
 """
 import argparse
+import collections
 import json
 import os
 import subprocess
@@ -60,6 +62,7 @@ def parse():
     ap.add_argument("--configs", default=os.environ.get("MFR_BENCH_CONFIGS", "C1,C3,C4,C5"), help="extra BASELINE configs to measure ('' = none)")
     ap.add_argument("--stream-pairs", type=int, default=10000, help="length of the C4 pair stream")
     ap.add_argument("--no-siblings", action="store_true", help="skip the tf32 / fp32x3 runs of the headline workload")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the poses of the last timed step of the headline run as DIR/<name>.npy")
     return ap.parse_args()
 
 
@@ -245,9 +248,10 @@ class Harness:
         h = self.h
         return pipe.submit_host(*[[h[k][i] for i in idx] for k in ("g0", "g1", "d0", "d1", "K", "K")])
 
-    def timed(self, pipe, eng, submit, n_batches, warm_batches, gather_at_end=False, sampler=None):
-        """CUDA-event time (ms, max over ranks) of `n_batches` engine batches through `pipe`, after `warm_batches`.
-        `sampler` (ClockSampler) runs during the timed region only (not during the warm-up)."""
+    def timed(self, pipe, eng, submit, n_batches, warm_batches, gather_at_end=False, sampler=None, keep=1):
+        """CUDA-event time (ms, max over ranks) of `n_batches` engine batches through `pipe`, after `warm_batches`, and
+        the results of the last `keep` of them, oldest first. `sampler` (ClockSampler) runs during the timed region only
+        (not during the warm-up)."""
         torch, dist = self.torch, self.dist
         for b in range(warm_batches):
             submit(b)
@@ -258,9 +262,13 @@ class Harness:
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         with torch.cuda.stream(eng.stream):
             e0.record()
+        tail = collections.deque(maxlen=keep)
         for b in range(n_batches):
-            submit(warm_batches + b)
+            r = submit(warm_batches + b)             # the result of the batch submitted before this one
+            if r is not None:
+                tail.append(r)
         last = pipe.drain()                          # the timed region ends when the last batch's poses are on the host
+        tail.append(last)
         if gather_at_end and self.world > 1:
             R, t, n = last
             with torch.cuda.stream(eng.stream):
@@ -276,7 +284,7 @@ class Harness:
         ms = torch.tensor([e0.elapsed_time(e1)], device=self.dev)
         if self.world > 1:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
-        return float(ms.item()), last
+        return float(ms.item()), list(tail)
 
 
 def matches_of(eng, i0, i1):
@@ -347,7 +355,8 @@ def run_ours(args):
     in_bytes = sum(int(np.prod(hs.h[k].shape[1:])) * hs.h[k].element_size() * B for k in ("g0", "g1", "d0", "d1", "K", "K")) * micro
     out_bytes = int(pipe.slots[0]["rec_host"].numel() * 4) * micro
     clk, clk2 = ClockSampler(hs.local_rank), ClockSampler(hs.local_rank)
-    ms_res, last = hs.timed(pipe, eng, lambda b: hs.submit_resident(pipe, eng, b), K * micro, Wm * micro, gather_at_end=True, sampler=clk)
+    ms_res, last_step = hs.timed(pipe, eng, lambda b: hs.submit_resident(pipe, eng, b), K * micro, Wm * micro, gather_at_end=True,
+                                 sampler=clk, keep=micro)
     clocks = clk.summary()
     ms_e2e, _ = hs.timed(pipe, eng, lambda b: hs.submit_host(pipe, b), K * micro, Wm * micro, sampler=clk2)
     clocks_e2e = clk2.summary()
@@ -470,7 +479,20 @@ def run_ours(args):
         dist.barrier()
         dist.destroy_process_group()
     if rank == 0:
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, last_step)
         print(json.dumps(result))
+
+
+def dump_outputs(out_dir, results):
+    """Writes the poses the pipeline handed out for the engine batches of one step, one row per pair in submission
+    order (row j of the b-th batch since the first warm-up batch is pool pair (b * batch + j) mod pool): R.npy [P,3,3],
+    t.npy [P,3] float32 and inliers.npy [P] (counts, as float32)."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    R, t, n = (torch.cat([r[k] for r in results]) for k in range(3))
+    for name, a in (("R", R), ("t", t), ("inliers", n)):
+        np.save(os.path.join(out_dir, name + ".npy"), a.numpy().astype(np.float32))
 
 
 # ------------------------------------------------------------------------------------------------

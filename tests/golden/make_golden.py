@@ -14,7 +14,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__)
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 import mfr_b200  # noqa: E402,F401
-from helpers import spsg_real_cases  # noqa: E402
+from helpers import METRICS_K, loftr_module_case, metrics_cases, metrics_checksum, spsg_real_cases  # noqa: E402
 from mfr_b200 import synth  # noqa: E402
 from oracle import ref_import, loftr_oracle  # noqa: E402
 
@@ -195,9 +195,70 @@ def make_spsg_real_golden():
     np.savez_compressed(os.path.join(HERE, "spsg_real_reference.npz"), **out)
 
 
+def make_loftr_module_golden():
+    """The reference LoFTR module with seeded weights (make_state_dict(3)) at coarse threshold 0: the full
+    confidence matrix and the matches."""
+    LoFTR, default_cfg = ref_import.load_loftr()
+    sd = loftr_oracle.make_state_dict(3)
+    m = LoFTR(config=default_cfg).eval()
+    m.load_state_dict({k: v.clone() for k, v in sd.items()}, strict=False)
+    m.coarse_matching.thr = 0.0
+    i0, i1 = loftr_module_case()
+    with torch.no_grad():
+        b = {"image0": i0, "image1": i1}
+        m(b)
+    out = {"checksum": checksum(i0.numpy(), i1.numpy()), "conf_matrix": b["conf_matrix"].numpy()}
+    for k in ("i_ids", "j_ids", "mkpts1_f"):
+        out[k] = b[k].numpy()
+    np.savez_compressed(os.path.join(HERE, "loftr_module_reference.npz"), **out)
+    print("loftr module golden: M =", len(out["i_ids"]))
+
+
+def make_metrics_golden():
+    """The reference's benchmark/metrics.py MetricManager and benchmark/utils.py precision_recall on
+    metrics_cases(); transforms3d (not installed) is stood in for by the oracle's restatement of the four
+    quaternion helpers it provides."""
+    import types
+    from oracle import metrics_oracle as mo
+    t3d = types.ModuleType("transforms3d"); tq = types.ModuleType("transforms3d.quaternions"); te = types.ModuleType("transforms3d.euler")
+    for n in ("quat2mat", "qmult", "qinverse", "rotate_vector", "axangle2quat"):
+        setattr(tq, n, getattr(mo, n))
+    te.euler2quat = mo.euler2quat
+    t3d.quaternions, t3d.euler = tq, te
+    sys.modules.update({"transforms3d": t3d, "transforms3d.quaternions": tq, "transforms3d.euler": te})
+    sys.path.insert(0, ref_import.REF)
+    from benchmark.metrics import Inputs, MetricManager
+    from benchmark.utils import precision_recall
+    cases = metrics_cases()
+    res = {"trans_err": [], "rot_err": [], "reproj_err": [], "confidence": []}
+    mm = MetricManager()
+    for qg, tg, qe, te_, conf in cases:
+        mm(Inputs(q_gt=qg, t_gt=tg, q_est=qe, t_est=te_, confidence=conf, K=METRICS_K, W=540, H=720), res)
+    out = {k: np.asarray(v, np.float64) for k, v in res.items()}
+    out["checksum"] = metrics_checksum(cases)
+    tp = (out["trans_err"] < 0.25) * (out["rot_err"] < 5)
+    out["precision"], out["recall"], out["ap"] = [np.asarray(x, np.float64) for x in precision_recall(out["confidence"].tolist(), tp, 3)]
+    np.savez_compressed(os.path.join(HERE, "metrics_reference.npz"), **out)
+    print("metrics golden:", len(cases), "poses, AP", float(out["ap"]))
+
+
+README_PAIR = ("scene0711_00_frame-001680.jpg", "scene0711_00_frame-001995.jpg")
+
+
+def make_readme_pair_fixtures():
+    """The SuperGlue README's ScanNet sample pair (1296x968 camera JPEGs), re-encoded at quality 75 to keep the
+    repository small; they exercise the GPU JPEG loader on real photographs."""
+    import cv2
+    src = os.path.join(ref_import.FMB, "SuperGlue", "assets", "scannet_sample_images")
+    for n in README_PAIR:
+        im = cv2.imread(os.path.join(src, n), cv2.IMREAD_COLOR)
+        assert cv2.imwrite(os.path.join(HERE, n), im, [cv2.IMWRITE_JPEG_QUALITY, 75])
+    print("readme pair fixtures:", ", ".join(README_PAIR))
+
+
 if __name__ == "__main__":
-    assert ref_import.available(), "needs /root/reference"
-    which = sys.argv[1:] or ["pose", "loftr", "fullres", "spsg", "spsg_real"]
+    assert ref_import.available(), "needs the reference tree (MFR_REFERENCE)"
+    which = sys.argv[1:] or ["pose", "loftr", "fullres", "spsg", "spsg_real", "loftr_module", "metrics", "images"]
     if "pose" in which:
         make_pose_golden()
     if "loftr" in which:
@@ -208,3 +269,9 @@ if __name__ == "__main__":
         make_spsg_golden()
     if "spsg_real" in which:
         make_spsg_real_golden()
+    if "loftr_module" in which:
+        make_loftr_module_golden()
+    if "metrics" in which:
+        make_metrics_golden()
+    if "images" in which:
+        make_readme_pair_fixtures()

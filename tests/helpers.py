@@ -48,6 +48,36 @@ def vec_angle(a, b):
     return float(np.arccos(np.clip(a @ b / (np.linalg.norm(a) * np.linalg.norm(b)), -1.0, 1.0)))
 
 
+def loftr_module_case():
+    """Seeded 96x64 input and its shifted copy (tests/golden/make_golden.py: make_loftr_module_golden)."""
+    import torch
+    g = torch.Generator().manual_seed(5)
+    i0 = torch.rand(1, 1, 96, 64, generator=g)
+    return i0, torch.roll(i0, (8, 8), (2, 3))
+
+
+METRICS_K = np.array([[590.0, 0, 270.0], [0, 590.0, 360.0], [0, 0, 1]])
+
+
+def metrics_cases():
+    """40 seeded (q_gt, t_gt, q_est, t_est, confidence) pose estimates around ground truth, drawn with the oracle's
+    restatement of the transforms3d helpers (tests/golden/make_golden.py: make_metrics_golden)."""
+    from oracle import metrics_oracle as mo
+    rng = np.random.default_rng(1)
+    cases = []
+    for _ in range(40):
+        qg = mo.euler2quat(*rng.uniform(0, 2 * np.pi, 3))
+        qe = mo.qmult(qg, mo.axangle2quat(rng.uniform(-1, 1, 3), rng.uniform(0, 0.3)))
+        tg = rng.normal(0, 1, 3)
+        te = tg + rng.normal(0, 0.2, 3)
+        cases.append((qg, tg, qe, te, float(rng.integers(0, 50))))
+    return cases
+
+
+def metrics_checksum(cases):
+    return checksum(*[np.concatenate([qg, tg, qe, te, [conf]]) for qg, tg, qe, te, conf in cases])
+
+
 # ---- BASELINE-configuration LoFTR case (tests/golden/make_golden.py: make_loftr_fullres_golden) ----
 FULLRES_CASES = [("dense", 0.0), ("functional", 0.2), ("functional_dense", 0.2)]
 FULLRES_SEEDS = (1000, 1001)

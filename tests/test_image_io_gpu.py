@@ -7,8 +7,7 @@ import numpy as np
 import pytest
 import torch
 
-from helpers import synth
-from oracle import build_ref
+from helpers import GOLDEN, synth
 
 pytestmark = pytest.mark.gpu
 
@@ -90,13 +89,13 @@ def test_jpeg_decode_and_plugins(tmp_path):
     assert out.shape[1] == 4
 
 
-@pytest.mark.skipif(not build_ref.available(), reason="oracle/_ref assets not staged")
 def test_readme_pair_through_the_gpu_loader():
-    """The SuperGlue README sample pair read by the GPU loader = the arrays the golden vectors were made from (up to the
-    JPEG decoders' +-2 gray levels): same keypoint counts within a few detections."""
+    """Camera JPEGs (the SuperGlue README's 1296x968 ScanNet sample pair, stored re-encoded at quality 75) read by the GPU
+    loader at the 640x480 of the README's known-answer test = OpenCV's decode and float resize up to the JPEG decoders'
+    +-2 gray levels."""
     from mfr_b200 import image_io
     for n in ("scene0711_00_frame-001680.jpg", "scene0711_00_frame-001995.jpg"):
-        path = build_ref.data_dir() + "/" + n
+        path = GOLDEN + "/" + n
         got = image_io.read_image(path, (640, 480), True).cpu().numpy()
         ref = cv2.resize(cv2.imread(path, cv2.IMREAD_GRAYSCALE).astype("float32"), (640, 480)) / 255.0
         assert np.abs(got - ref).max() < 3.5 / 255 and np.abs(got - ref).mean() < 0.5 / 255

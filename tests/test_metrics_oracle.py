@@ -1,18 +1,15 @@
 """The metrics oracle (oracle/metrics_oracle.py) against the reference's OWN tests for this code
 (benchmark/test_metrics.py: properties of trans_err / rot_err / reproj_err and the known-answer vectors of
-test_projection, replayed here with seeded randomness), and — when /root/reference is mounted — against the reference
-module itself on random poses (transforms3d, which the reference imports and this image lacks, is stood in for by the
+test_projection, replayed here with seeded randomness), and against stored outputs of the reference module itself on
+random poses (tests/golden/make_golden.py; transforms3d, which the reference imports, is stood in for there by the
 oracle's restatement of its four quaternion helpers)."""
-import sys
-import types
-
 import numpy as np
 import pytest
 
-from helpers import ROOT  # noqa: F401
-from oracle import metrics_oracle as mo, ref_import
+from helpers import GOLDEN, METRICS_K, metrics_cases, metrics_checksum
+from oracle import metrics_oracle as mo
 
-K0 = np.array([[590.0, 0, 270.0], [0, 590.0, 360.0], [0, 0, 1]])
+K0 = METRICS_K
 
 
 def _rq(rng):
@@ -55,44 +52,20 @@ def test_precision_recall_small_case():
     assert np.isclose(ap, 0.2 * 0.75 + 0.4 * 2 / 3 + 0.2 * 1.0)
 
 
-@pytest.mark.skipif(not ref_import.available(), reason="needs /root/reference")
 def test_oracle_equals_reference_module():
-    t3d = types.ModuleType("transforms3d"); tq = types.ModuleType("transforms3d.quaternions"); te = types.ModuleType("transforms3d.euler")
-    for n in ("quat2mat", "qmult", "qinverse", "rotate_vector", "axangle2quat"):
-        setattr(tq, n, getattr(mo, n))
-    te.euler2quat = mo.euler2quat
-    t3d.quaternions, t3d.euler = tq, te
-    saved = {k: sys.modules.get(k) for k in ("transforms3d", "transforms3d.quaternions", "transforms3d.euler")}
-    sys.modules.update({"transforms3d": t3d, "transforms3d.quaternions": tq, "transforms3d.euler": te})
-    sys.path.insert(0, ref_import.REF)
-    try:
-        from benchmark.metrics import Inputs, MetricManager
-        from benchmark.utils import precision_recall
-        rng = np.random.default_rng(1)
-        res = {"trans_err": [], "rot_err": [], "reproj_err": [], "confidence": []}
-        mm = MetricManager()
-        ours = {k: [] for k in res}
-        for _ in range(40):
-            qg = _rq(rng)
-            qe = mo.qmult(qg, mo.axangle2quat(rng.uniform(-1, 1, 3), rng.uniform(0, 0.3)))
-            tg = rng.normal(0, 1, 3); te_ = tg + rng.normal(0, 0.2, 3)
-            conf = float(rng.integers(0, 50))
-            mm(Inputs(q_gt=qg, t_gt=tg, q_est=qe, t_est=te_, confidence=conf, K=K0, W=540, H=720), res)
-            m = mo.pose_metrics(qg, tg, qe, te_, K0, 540, 720)
-            for k in ("trans_err", "rot_err", "reproj_err"):
-                ours[k].append(m[k])
-            ours["confidence"].append(conf)
-        for k in res:
-            assert np.allclose(res[k], ours[k], rtol=1e-10, atol=1e-10), k
-        tp = (np.array(ours["trans_err"]) < 0.25) * (np.array(ours["rot_err"]) < 5)
-        a, b = precision_recall(ours["confidence"], tp, 3), mo.precision_recall(ours["confidence"], tp, 3)
-        assert np.allclose(a[0], b[0]) and np.allclose(a[1], b[1]) and np.isclose(a[2], b[2])
-    finally:
-        sys.path.remove(ref_import.REF)
-        for k, v in saved.items():
-            if v is None:
-                sys.modules.pop(k, None)
-            else:
-                sys.modules[k] = v
-        for k in [k for k in sys.modules if k == "benchmark" or k.startswith("benchmark.")]:
-            sys.modules.pop(k)
+    """benchmark/metrics.py MetricManager and benchmark/utils.py precision_recall of the reference, stored in
+    tests/golden/metrics_reference.npz, against the oracle on the same 40 seeded poses."""
+    G = np.load(GOLDEN + "/metrics_reference.npz")
+    cases = metrics_cases()
+    assert metrics_checksum(cases) == pytest.approx(float(G["checksum"]), rel=1e-12)
+    ours = {k: [] for k in ("trans_err", "rot_err", "reproj_err", "confidence")}
+    for qg, tg, qe, te_, conf in cases:
+        m = mo.pose_metrics(qg, tg, qe, te_, K0, 540, 720)
+        for k in ("trans_err", "rot_err", "reproj_err"):
+            ours[k].append(m[k])
+        ours["confidence"].append(conf)
+    for k in ours:
+        assert np.allclose(G[k], ours[k], rtol=1e-10, atol=1e-10), k
+    tp = (np.array(ours["trans_err"]) < 0.25) * (np.array(ours["rot_err"]) < 5)
+    b = mo.precision_recall(ours["confidence"], tp, 3)
+    assert np.allclose(G["precision"], b[0]) and np.allclose(G["recall"], b[1]) and np.isclose(G["ap"], b[2])

@@ -1,85 +1,63 @@
-"""Live cross-check of the oracle restatements against the reference modules (build container only;
-skipped where /root/reference does not exist, e.g. on the GPU box)."""
+"""The oracle restatements against outputs of the reference modules themselves, stored under tests/golden/
+(tests/golden/make_golden.py regenerates them from the reference tree)."""
 import numpy as np
 import pytest
 import torch
 
-from helpers import pose_case
-from oracle import ref_import, loftr_oracle, pose_solver_oracle as po
-
-pytestmark = pytest.mark.skipif(not ref_import.available(), reason="reference tree not mounted")
+from helpers import GOLDEN, checksum, loftr_module_case, pose_case, spsg_real_cases
+from oracle import build_ref, loftr_oracle, pose_solver_oracle as po
 
 
 def test_pose_solver_module_matches_oracle():
-    model = ref_import.load_model_module()
+    """The reference's FeatureMatchingModel (precomputed matches) with the metric essential-matrix and the PnP solver."""
+    G = np.load(GOLDEN + "/pose_solver_reference.npz")
     c = pose_case(1)
-    corr = np.concatenate([c["kpts0"], c["kpts1"]], 1)[None].astype(np.float64)
-    np.savez_compressed("/tmp/_mfr_live_corr.npz", correspondences=corr)
+    assert checksum(c["kpts0"], c["kpts1"], c["depth0"], c["depth1"]) == pytest.approx(float(G["c1_checksum"]), rel=0, abs=1e-6)
     for solver in ("EssentialMatrixMetric", "PNP"):
-        cfg = ref_import.Cfg.wrap(dict(FEATURE_MATCHING="Precomputed", DEBUG=False, POSE_SOLVER=solver,
-                                       MATCHES_FILE_PATH="/tmp/_mfr_live_corr.npz",
-                                       EMAT_RANSAC=dict(PIX_THRESHOLD=2.0, SCALE_THRESHOLD=0.1, CONFIDENCE=0.9999),
-                                       PNP=dict(RANSAC_ITER=1000, REPROJECTION_INLIER_THRESHOLD=3, CONFIDENCE=0.9999),
-                                       DATASET=dict(PAIRS_TXT=dict(TEST=None))))
-        m = model.FeatureMatchingModel(cfg)
-        data = {"depth0": torch.from_numpy(c["depth0"])[None], "depth1": torch.from_numpy(c["depth1"])[None],
-                "K_color0": torch.from_numpy(c["K_color0"])[None], "K_color1": torch.from_numpy(c["K_color1"])[None],
-                "pair_id": torch.tensor([0])}
-        R, t = m(data)
         if solver == "PNP":
             Ro, to, no = po.pnp_solver(c["kpts0"], c["kpts1"], c["depth0"], c["K_color0"], c["K_color1"], 1000, 3, 0.9999)
         else:
             Ro, to, no = po.essential_matrix_metric_solver(c["kpts0"], c["kpts1"], c["depth0"], c["depth1"],
                                                            c["K_color0"], c["K_color1"], 2.0, 0.9999, 0.1)
-        np.testing.assert_allclose(R[0].numpy(), np.float32(Ro), atol=1e-6)
-        np.testing.assert_allclose(t[0, 0].numpy(), np.float32(to).ravel(), atol=1e-6)
-        assert data["inliers"] == no
+        np.testing.assert_allclose(G[f"c1_{solver}_R"], np.float32(Ro), atol=1e-6)
+        np.testing.assert_allclose(G[f"c1_{solver}_t"], np.float32(to).ravel(), atol=1e-6)
+        assert int(G[f"c1_{solver}_inliers"]) == no
 
 
 def test_loftr_module_matches_oracle():
-    LoFTR, default_cfg = ref_import.load_loftr()
+    G = np.load(GOLDEN + "/loftr_module_reference.npz")
     sd = loftr_oracle.make_state_dict(3)
-    m = LoFTR(config=default_cfg).eval()
-    missing = m.load_state_dict({k: v.clone() for k, v in sd.items()}, strict=False)
-    assert not missing.unexpected_keys
-    assert all("num_batches_tracked" in k for k in missing.missing_keys)
-    g = torch.Generator().manual_seed(5)
-    i0 = torch.rand(1, 1, 96, 64, generator=g)
-    i1 = torch.roll(i0, (8, 8), (2, 3))
-    m.coarse_matching.thr = 0.0
+    i0, i1 = loftr_module_case()
+    assert checksum(i0.numpy(), i1.numpy()) == pytest.approx(float(G["checksum"]), abs=1e-6)
     with torch.no_grad():
-        b = {"image0": i0, "image1": i1}
-        m(b)
         o = loftr_oracle.loftr_forward(i0, i1, sd, {"thr": 0.0}, True)
-    assert torch.equal(b["i_ids"], o["i_ids"]) and torch.equal(b["j_ids"], o["j_ids"])
-    torch.testing.assert_close(b["conf_matrix"], o["conf"], rtol=1e-5, atol=1e-12)
-    torch.testing.assert_close(b["mkpts1_f"], o["mkpts1_f"], atol=2e-4, rtol=0)
+    np.testing.assert_array_equal(o["i_ids"].numpy(), G["i_ids"])
+    np.testing.assert_array_equal(o["j_ids"].numpy(), G["j_ids"])
+    torch.testing.assert_close(torch.from_numpy(G["conf_matrix"]), o["conf"], rtol=1e-5, atol=1e-12)
+    torch.testing.assert_close(torch.from_numpy(G["mkpts1_f"]), o["mkpts1_f"], atol=2e-4, rtol=0)
 
 
+@pytest.mark.skipif(not build_ref.available(), reason="the reference's pretrained SuperPoint / SuperGlue weights are not staged in oracle/_ref")
 def test_spsg_modules_match_oracle_with_real_weights():
-    """The in-tree SuperPoint/SuperGlue weights on an in-tree ScanNet sample pair: identical keypoints,
-    descriptors and matches (the reference README's known-answer pair, SuperGlue/README.md:121-127)."""
-    import cv2
+    """The pretrained SuperPoint/SuperGlue weights on the reference README's known-answer ScanNet pair
+    (SuperGlue/README.md:121-127): identical keypoints, descriptors and matches."""
     from oracle import spsg_oracle as so
-    SuperPoint, SuperGlue, Matching = ref_import.load_superglue()
-    wdir = ref_import.FMB + "/SuperGlue/models/weights/"
-    sp_sd = torch.load(wdir + "superpoint_v1.pth", map_location="cpu")
-    sg_sd = torch.load(wdir + "superglue_indoor.pth", map_location="cpu")
-    adir = ref_import.FMB + "/SuperGlue/assets/scannet_sample_images/"
-
-    def load(n):
-        im = cv2.resize(cv2.imread(adir + n, cv2.IMREAD_GRAYSCALE).astype("float32"), (640, 480))
-        return torch.from_numpy(im / 255.0).float()[None, None]
-
-    i0, i1 = load("scene0711_00_frame-001680.jpg"), load("scene0711_00_frame-001995.jpg")
-    m = Matching({"superpoint": {"nms_radius": 4, "keypoint_threshold": 0.005, "max_keypoints": 1024},
-                  "superglue": {"weights": "indoor", "sinkhorn_iterations": 20, "match_threshold": 0.2}}).eval()
+    G = np.load(GOLDEN + "/spsg_real_reference.npz")
+    wdir = build_ref.weights_dir()
+    sp_sd = torch.load(wdir + "/superpoint_v1.pth", map_location="cpu")
+    sg_sd = torch.load(wdir + "/superglue_indoor.pth", map_location="cpu")
+    name, i0, i1 = spsg_real_cases()[0]
+    assert name == "readme"
+    assert checksum(i0.numpy(), i1.numpy()) == pytest.approx(float(G["readme_checksum"]), rel=1e-6)
     with torch.no_grad():
-        pred = m({"image0": i0, "image1": i1})
         k0, s0, d0 = so.superpoint(i0, sp_sd)
         k1, s1, d1 = so.superpoint(i1, sp_sd)
         m0, ms0 = so.superglue(k0, s0, d0, k1, s1, d1, 480, 640, sg_sd)
-    assert torch.equal(k0, pred["keypoints0"][0]) and torch.equal(k1, pred["keypoints1"][0])
-    torch.testing.assert_close(d0, pred["descriptors0"][0], atol=1e-6, rtol=0)
-    assert torch.equal(m0, pred["matches0"][0]) and int((m0 > -1).sum()) > 100
-    torch.testing.assert_close(ms0, pred["matching_scores0"][0], atol=1e-5, rtol=0)
+    np.testing.assert_array_equal(k0.numpy(), G["readme_keypoints0"])
+    np.testing.assert_array_equal(k1.numpy(), G["readme_keypoints1"])
+    np.testing.assert_allclose(d0[::8, ::4].numpy(), G["readme_descriptors0_sample"], atol=1e-6, rtol=0)
+    np.testing.assert_array_equal(m0.numpy(), G["readme_matches0"])
+    assert int((m0 > -1).sum()) > 100
+    # the stored scores may come from a CPU with other vector instructions: after 18 attention layers and 20 Sinkhorn
+    # iterations in fp32 they differ by up to 1.0e-5 across such hosts (they are bit-identical on the host that made them)
+    np.testing.assert_allclose(ms0.numpy(), G["readme_matching_scores0"], atol=2e-5, rtol=0)
